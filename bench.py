@@ -15,6 +15,11 @@ context is NOT tied to --steps:
      (per window: CUDA events on the decoder's stream, max over ranks);
   4. `by_position` adds tokens/s in short windows at positions 1, 256 and 1023.
 
+--dump-outputs DIR writes what the timed path returned at its last timed step (last window of the last
+repetition) as DIR/logits.npy (float32 [vocab]) and DIR/next_token.npy (float64 [1], the greedy id).
+Weights and token inputs are seeded, so runs with the same arguments see identical inputs and two builds
+can be compared output for output.
+
   value   device-resident loop: tokens fed back on the GPU, no host round trip inside a window.
   e2e     the same positions through the reference-facing call kllm_decoder_step() with HOST
           buffers: per step the token id + position go host->device (pinned, 16 B), the greedy id
@@ -32,8 +37,9 @@ the fp32 Llama-2-7B of configs[4] is measured in the same run and reported under
 
 --impl reference       the reference's CPU implementation of the path (oracle port; the reference's
                        CMake build needs Armadillo/glog/gtest/sentencepiece, none installed).
---impl reference-cuda  the reference's own CUDA kernels + model code (oracle/_ref, compiled from
-                       /root/reference for sm_100a) timed on the same GPU: the "reference GPU" row.
+--impl reference-cuda  the reference's own CUDA kernels + model code (oracle/_ref, compiled from the
+                       checkout KUIPER_REFERENCE_DIR names, for sm_100a) timed on the same GPU: the
+                       "reference GPU" row.
 """
 from __future__ import annotations
 
@@ -89,6 +95,8 @@ def parse_args():
     ap.add_argument("--no-secondary", action="store_true", help="N>1: skip the fp32 Llama-2-7B line (configs[4])")
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="budget of the cpu_baseline leg")
     ap.add_argument("--seed", type=int, default=None)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the timed path's outputs of its last step to DIR/*.npy (--impl ours)")
     return ap.parse_args()
 
 
@@ -488,12 +496,13 @@ class Bench:
             if got != self.ids[start:start + n]:
                 raise SystemExit(f"window at position {start} ({'e2e' if e2e else 'device loop'}) produced token ids "
                                  "that differ from the pre-pass")
+            self.last_ids = got
             out.append(e0.elapsed_time(e1))
         return self._max_over_ranks(out)
 
     def run(self):
         args, shape = self.args, self.shape
-        K = min(args.steps, shape.seq_len)
+        K = args.steps
         ctx = min(CONTEXT, shape.seq_len)
         windows = plan_windows(K, ctx)
         self.prepass()
@@ -507,6 +516,10 @@ class Bench:
             ms = self.time_windows(windows)
             totals.append(sum(ms)); per_window.append(ms)
         t_wall1 = time.time()
+        if args.dump_outputs:
+            # what a caller of the timed path holds after its last step (read outside the timed region)
+            import numpy as np
+            self.last_step = {"logits": self.dec.logits(), "next_token": np.array([self.last_ids[-1]], np.float64)}
         launches = (self.lib.kllm_launch_count() - launches0) // reps
         clocks = sampler.stop(t_wall0, t_wall1) if sampler else None
         ms_total = statistics.median(totals)
@@ -585,6 +598,11 @@ def run_ours(args, rank, world):
     b = Bench(args, rank, world, args.workload, stream, lib)
     shape = b.shape
     res = b.run()
+    if rank == 0 and args.dump_outputs:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in b.last_step.items():
+            np.save(os.path.join(args.dump_outputs, f"{name}.npy"), a)
     line = None
     if rank == 0:
         line = {
@@ -662,6 +680,10 @@ def run_ours(args, rank, world):
 
 def main():
     args = parse_args()
+    if args.steps < 1:
+        raise SystemExit("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        raise SystemExit("--dump-outputs applies to --impl ours")
     # ONE JSON line on stdout: libraries that chat on fd 1 (NCCL prints its version there) go to stderr
     global _REAL_STDOUT
     sys.stdout.flush()
@@ -681,6 +703,10 @@ def main():
         args.workload = default_workload(args.gpus)
     if args.seed is None:
         args.seed = SEEDS.get(args.workload, 1234)
+    from kuiperllama_b200 import SHAPES
+    if args.impl == "ours" and args.steps > SHAPES[args.workload].seq_len:
+        raise SystemExit(f"--steps {args.steps} exceeds the context of {SHAPES[args.workload].name} "
+                         f"({SHAPES[args.workload].seq_len} positions)")
     if args.impl == "reference":
         run_reference(args, rank, world)
     elif args.impl == "reference-cuda":

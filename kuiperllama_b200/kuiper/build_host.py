@@ -14,7 +14,18 @@ from pathlib import Path
 
 HERE = Path(__file__).resolve().parent
 VARIANTS = {"llama2": [], "qwen2": ["-DQWEN2_SUPPORT=ON"], "llama3": ["-DLLAMA3_SUPPORT=ON"]}
-REFERENCE = Path("/root/reference")
+
+
+def reference_checkout() -> Path | None:
+    """The reference checkout named by KUIPER_REFERENCE_DIR whose demo programs are built unchanged,
+    or None when the variable is unset or the demo sources cannot be read."""
+    d = os.environ.get("KUIPER_REFERENCE_DIR")
+    if not d:
+        return None
+    try:
+        return Path(d) if (Path(d) / "demo" / "main.cpp").is_file() else None
+    except OSError:
+        return None
 
 
 def build_dir(variant: str) -> Path:
@@ -37,8 +48,9 @@ def build(variant: str = "llama2", verbose: bool = False) -> Path:
            "-DCMAKE_CXX_COMPILER=/usr/bin/g++", *VARIANTS[variant]]
     if shutil.which("ninja"):
         cfg += ["-G", "Ninja"]
-    if (REFERENCE / "demo" / "main.cpp").exists():
-        cfg.append(f"-DKUIPER_REFERENCE_DIR={REFERENCE}")
+    reference = reference_checkout()
+    if reference is not None:
+        cfg.append(f"-DKUIPER_REFERENCE_DIR={reference}")
     quiet = {} if verbose else {"stdout": subprocess.PIPE, "stderr": subprocess.STDOUT}
     for cmd in (cfg, [cmake, "--build", str(out), "-j", str(min(32, os.cpu_count() or 4))]):
         r = subprocess.run(cmd, text=True, **quiet)

@@ -20,9 +20,20 @@ HERE = Path(__file__).resolve().parent
 ORACLE_SO = HERE / "_build" / "liboracle.so"
 REF_SO = HERE / "_ref" / "libkuiper_ref.so"
 REF_QWEN_SO = HERE / "_ref" / "libkuiper_ref_qwen2_kernels.so"
-REFERENCE_TREE = Path("/root/reference")
 
 FLAVOURS = {"llama2": 0, "llama3": 1, "qwen2": 2, "qwen2file": 3}
+
+
+def reference_tree() -> Path | None:
+    """The reference checkout named by KUIPER_REFERENCE_DIR, or None when the variable is unset or
+    the tree cannot be read (an unreadable path is the same as an absent one)."""
+    d = os.environ.get("KUIPER_REFERENCE_DIR")
+    if not d:
+        return None
+    try:
+        return Path(d) if (Path(d) / "kuiper" / "source").is_dir() else None
+    except OSError:
+        return None
 
 
 def build_oracle() -> Path:
@@ -31,11 +42,12 @@ def build_oracle() -> Path:
 
 
 def build_ref(jobs: int = 8) -> bool:
-    """Compile oracle/_ref from /root/reference when that tree is present (build container);
-    on the GPU box the prebuilt .so files that travelled with the snapshot are used."""
-    if not REFERENCE_TREE.is_dir():
+    """Compile oracle/_ref from the reference checkout when KUIPER_REFERENCE_DIR names one;
+    otherwise report whether an earlier build of oracle/_ref is present."""
+    tree = reference_tree()
+    if tree is None:
         return REF_SO.exists()
-    subprocess.check_call(["make", "-s", f"-j{jobs}", "-C", str(HERE), "ref"])
+    subprocess.check_call(["make", "-s", f"-j{jobs}", "-C", str(HERE), f"REF={tree}", "ref"])
     return True
 
 
@@ -261,7 +273,7 @@ class RefCuda:
     def __init__(self, flavour="llama2"):
         so = REF_SO if flavour == "llama2" else REF_QWEN_SO
         if not so.exists():
-            raise FileNotFoundError(f"{so} not built (run `make -C oracle ref` where /root/reference exists)")
+            raise FileNotFoundError(f"{so} not built (run `make -C oracle REF=<reference checkout> ref`)")
         L = ctypes.CDLL(str(so))
         vp = c_void_p
         L.kref_flavour.restype = c_char_p

@@ -5,6 +5,7 @@ import json
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 from conftest import ROOT
@@ -71,3 +72,27 @@ def test_default_workload_follows_the_metric():
     import torch
     if not torch.cuda.is_available():
         assert bench.default_workload(1) == "tinyllama-1.1b"
+
+
+def test_steps_beyond_the_models_context_are_refused():
+    r = _run("--workload", "small", "--steps", "161", "--warmup", "3", "--no-cpu-baseline")
+    assert r.returncode != 0 and r.stdout.strip() == "" and "exceeds the context" in r.stderr
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_the_last_timed_step_and_repeat(tmp_path):
+    """--dump-outputs DIR: the logits and greedy id of the last timed step, identical from run to run
+    (same arguments, same seeded inputs); --steps is the number of timed positions."""
+    outs = []
+    for i in range(2):
+        d = tmp_path / str(i)
+        r = _run("--workload", "small", "--steps", "12", "--warmup", "3", "--reps", "1", "--no-exact",
+                 "--no-cpu-baseline", "--dump-outputs", str(d))
+        assert r.returncode == 0, r.stderr
+        lines = [l for l in r.stdout.splitlines() if l.strip()]
+        assert len(lines) == 1 and json.loads(lines[0])["steps"] == 12
+        logits, tok = np.load(d / "logits.npy"), np.load(d / "next_token.npy")
+        assert logits.dtype == np.float32 and logits.shape == (4096,)
+        assert tok.dtype == np.float64 and tok.shape == (1,) and tok[0] == np.argmax(logits)
+        outs.append((logits, tok))
+    assert np.array_equal(outs[0][0], outs[1][0]) and np.array_equal(outs[0][1], outs[1][1])

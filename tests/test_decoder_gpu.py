@@ -2,7 +2,8 @@
   - the reference PyTorch logits committed under tests/golden (<= 1e-4, north-star tolerance),
   - the CPU oracle (same tolerance, identical greedy ids),
   - the reference's OWN CUDA model path run on this GPU (oracle/_ref): bit-identical logits,
-    KV cache and token ids -- including at BASELINE.json's full TinyLlama-1.1B size."""
+    KV cache and token ids -- including at BASELINE.json's full TinyLlama-1.1B size; live when
+    oracle/_ref is built, and always against its recorded outputs (tests/reference_outputs.py)."""
 import ctypes
 import os
 
@@ -12,6 +13,7 @@ import torch
 
 from conftest import GOLDEN
 from gpu_util import assert_bit_equal, sync
+from reference_outputs import check, live_reference
 
 pytestmark = pytest.mark.gpu
 
@@ -47,8 +49,7 @@ def load_decoder(path, quant=False, flavour="llama2", qkv_bias=None):
 
 @pytest.fixture(scope="module")
 def ref():
-    from oracle.binding import RefCuda
-    return RefCuda("llama2")
+    return live_reference("llama2")
 
 
 class RefModel:
@@ -96,13 +97,33 @@ def test_golden_logits(kllm_lib, oracle, name, quant, flavour, bias):
 def test_bit_exact_vs_reference_cuda_model_goldens(kllm_lib, ref, name, quant):
     g = np.load(GOLDEN / f"{name}.npz")
     dec, shape = load_decoder(GOLDEN / f"{name}.bin", quant)
-    rm = RefModel(ref, GOLDEN / f"{name}.bin", quant, shape.vocab_size)
+    rm = RefModel(ref, GOLDEN / f"{name}.bin", quant, shape.vocab_size) if ref else None
+    ids, logits, r_ids, r_logits = [], [], [], []
     for t, tok in enumerate(g["tokens"]):
-        nxt = dec.step(int(tok), t)
-        r_next, r_logits = rm.step(int(tok), t)
-        assert_bit_equal(dec.logits(), r_logits, f"{name} logits pos {t}")
-        assert nxt == r_next
-    rm.close(); dec.close()
+        ids.append(dec.step(int(tok), t))
+        logits.append(dec.logits())
+        if rm:
+            r_next, r_lg = rm.step(int(tok), t)
+            r_ids.append(r_next); r_logits.append(r_lg)
+    check(logits, r_logits if rm else None, f"model/{name}/logits", f"{name} logits [position, vocab]")
+    check(ids, r_ids if rm else None, f"model/{name}/ids", f"{name} token ids")
+    if rm:
+        rm.close()
+    dec.close()
+
+
+def _reference_free_run(ref, path, shape, steps):
+    """Greedy ids of `steps` free-running positions from token 1 and the last position's logits on the
+    reference's CUDA path (demo/main.cpp loop); (None, None) without a reference build."""
+    if not ref:
+        return None, None
+    rm = RefModel(ref, path, shape.group_size > 0, shape.vocab_size)
+    tok, ids = 1, []
+    for pos in range(steps):
+        tok, lg = rm.step(tok, pos, want_logits=(pos == steps - 1))
+        ids.append(tok)
+    rm.close()
+    return ids, lg
 
 
 def _synth_file(tmp_path, key, seed):
@@ -123,21 +144,17 @@ def test_free_running_decode_identical_to_reference_cuda(kllm_lib, ref, tmp_path
     from kuiperllama_b200 import Decoder
     shape, w, path = _synth_file(tmp_path, key, 100 + steps)
     dec = make_decoder(shape, w)
-    rm = RefModel(ref, path, shape.group_size > 0, shape.vocab_size)
     mine = dec.generate(1, 0, steps)
-    tok, theirs = 1, []
-    for pos in range(steps):
-        tok, lg = rm.step(tok, pos, want_logits=(pos == steps - 1))
-        theirs.append(tok)
-    assert mine == theirs
-    assert_bit_equal(dec.logits(), lg, f"{key}: logits after {steps} free-running steps")
+    theirs, lg = _reference_free_run(ref, path, shape, steps)
+    check(mine, theirs, f"free_run/{key}/{steps}/ids", f"{key}: token ids of {steps} free-running steps")
+    check(dec.logits(), lg, f"free_run/{key}/{steps}/logits", f"{key}: logits after {steps} free-running steps")
     # the host-buffer path (predict semantics) walks the same sequence
     tok = 1
     for pos in range(8):
         tok = dec.step(tok, pos)
-        assert tok == theirs[pos]
+        assert tok == mine[pos]
     assert dec.step(5, 3, is_prompt=True) == -1  # predict(..., is_prompt=true) returns -1
-    rm.close(); dec.close()
+    dec.close()
 
 
 @pytest.mark.parametrize("qkey", ["tiny-qwen", "small-qwen"])
@@ -192,16 +209,11 @@ def test_tinyllama_full_size_identical_to_reference_cuda(kllm_lib, ref, tmp_path
         write_checkpoint(path, shape, w)
         dec = make_decoder(shape, w)
         assert dec.engine == engine
-        rm = RefModel(ref, path, False, shape.vocab_size)
         steps = 256
         mine = dec.generate(1, 0, steps)
-        tok, theirs = 1, []
-        for pos in range(steps):
-            tok, lg = rm.step(tok, pos, want_logits=(pos == steps - 1))
-            theirs.append(tok)
-        assert mine == theirs
-        assert_bit_equal(dec.logits(), lg, "TinyLlama-1.1B logits after 256 steps")
-        rm.close()
+        theirs, lg = _reference_free_run(ref, path, shape, steps)
+        check(mine, theirs, "free_run/tinyllama-1.1b/256/ids", "TinyLlama-1.1B token ids of 256 steps")
+        check(dec.logits(), lg, "free_run/tinyllama-1.1b/256/logits", "TinyLlama-1.1B logits after 256 steps")
     finally:
         if os.path.exists(path):
             os.remove(path)
@@ -296,18 +308,12 @@ def test_llama2_7b_int8_full_size_identical_to_reference_cuda(kllm_lib, ref, eng
     shape = case["shape"]
     steps = 128
     if "ref_ids" not in case:
-        rm = RefModel(ref, case["path"], True, shape.vocab_size)
-        tok, theirs = 1, []
-        for pos in range(steps):
-            tok, lg = rm.step(tok, pos, want_logits=(pos == steps - 1))
-            theirs.append(tok)
-        rm.close()
-        case["ref_ids"], case["ref_logits"] = theirs, lg
+        case["ref_ids"], case["ref_logits"] = _reference_free_run(ref, case["path"], shape, steps)
     dec = make_decoder(shape, case["w"])
     assert dec.engine == engine
     mine = dec.generate(1, 0, steps)
-    assert mine == case["ref_ids"]
-    assert_bit_equal(dec.logits(), case["ref_logits"], "Llama-2-7B int8 logits after 128 steps")
+    check(mine, case["ref_ids"], "free_run/llama2-7b-int8/128/ids", "Llama-2-7B int8 token ids of 128 steps")
+    check(dec.logits(), case["ref_logits"], "free_run/llama2-7b-int8/128/logits", "Llama-2-7B int8 logits after 128 steps")
     # host-buffer path (predict semantics) at a late position reproduces the same id
     assert dec.step(mine[steps - 2], steps - 1) == mine[steps - 1]
     dec.close()

@@ -2,15 +2,14 @@
 (File name: sorts after the kernel / decoder suites, whose parity results it builds on.)
 
 not gpu: it builds with CMake, the reference's demo/main.cpp and demo/main_qwen.cpp compile and
-         link against it UNCHANGED (when /root/reference is present), and it fails loudly without
-         a GPU.
+         link against it UNCHANGED (when KUIPER_REFERENCE_DIR names a reference checkout), and it
+         fails loudly without a GPU.
 gpu:     decoding through model::LLama2Model / Qwen2Model (the demo's embedding -> fill_input ->
          predict loop) reproduces the committed goldens and is bit-identical to the C-ABI decoder,
          on the fused path and on the layer-by-layer op-registry path.
 """
 import subprocess
 import sys
-from pathlib import Path
 
 import numpy as np
 import pytest
@@ -20,7 +19,7 @@ from conftest import GOLDEN, ROOT as REPO
 sys.path.insert(0, str(REPO / "kuiperllama_b200" / "kuiper"))
 import build_host  # noqa: E402
 
-REFERENCE_PRESENT = (Path("/root/reference") / "demo" / "main.cpp").exists()
+REFERENCE_PRESENT = build_host.reference_checkout() is not None
 TOL = 1e-4
 
 
