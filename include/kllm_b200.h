@@ -21,6 +21,7 @@
  */
 #ifndef KLLM_B200_H_
 #define KLLM_B200_H_
+#include <stddef.h>
 #include <stdint.h>
 
 #ifdef __cplusplus
@@ -139,6 +140,23 @@ int kllm_gemv_fused(const kllm_gemv_job* job, void* stream);
 int kllm_gemm_tf32(const float* x, const float* w, float* out, int n_tokens, int in_dim, int out_dim,
                    void* stream);
 
+/* ---- batched prompt GEMM, int8 weights, on tcgen05.mma.kind::i8 (TOLERANCED: x rounded to 24-bit fixed point) ----
+ * out[n_tokens, out_dim] = x[n_tokens, in_dim] . (s (.) w)[out_dim, in_dim]^T with w int8 row-major and
+ * scales[(p*in_dim + i) / 64] the fp32 scale of weight (p, i) -- the int8 GEMV's formula with group_size 64
+ * (kllm_gemv_w8, export.py --version 3).  Each token's 64-element groups of x become step * q, step =
+ * max|x in group| * 2^-22, q = rint(x / step) as three int8 digit planes (the fast decode mode's definition,
+ * KLLM_NUMERICS_FAST); the int8 x int8 products of each group are exact in int32 on the tensor cores and are
+ * combined with s * step in fp32.  Only x is rounded, by at most 2^-23 of its group maximum, so results agree
+ * with the exact int8 GEMV to ~1e-6 relative (tests/test_prefill_w8_gpu.py states the bound), NOT bit for bit.
+ * `workspace`: caller-owned device memory of KLLM_GEMM_W8_WORKSPACE_BYTES(n_tokens, in_dim) bytes for the digit
+ * planes and steps (overwritten; do not share it between calls in flight on different streams).  No
+ * allocation, no synchronisation.  Limits: in_dim % 64 == 0 (else KLLM_E_UNSUPPORTED); x, w and workspace
+ * 16-byte aligned, scales and out 4-byte aligned (else KLLM_E_UNSUPPORTED); any n_tokens, out_dim >= 1. */
+#define KLLM_GEMM_W8_WORKSPACE_BYTES(n_tokens, in_dim) \
+  (3 * (size_t)(n_tokens) * (size_t)(in_dim) + 4 * ((size_t)(in_dim) / 64) * (((size_t)(n_tokens) + 63) / 64 * 64))
+int kllm_gemm_w8(const float* x, const int8_t* w, const float* scales, float* out, void* workspace, int n_tokens,
+                 int in_dim, int out_dim, void* stream);
+
 /* ---- tensor-parallel exchange --------------------------------------------------------------
  * Not in the reference (single GPU: llama3.cpp:118 pins device 0); SURVEY.md section 8e.  One
  * process per GPU; each owns a kllm_comm.  The decoder issues exactly two all-reduces per layer:
@@ -247,6 +265,14 @@ int kllm_decoder_prompt(kllm_decoder* dec, const int32_t* tokens_host, int32_t n
  * mantissa bits).  fp32 checkpoints on one GPU; KLLM_E_UNSUPPORTED otherwise (use kllm_decoder_prompt). */
 int kllm_decoder_prefill_tf32(kllm_decoder* dec, const int32_t* tokens_host, int32_t n_tokens, int32_t start_pos,
                               int32_t* next_host);
+/* TOLERANCED batched prefill for int8 checkpoints: the contract of kllm_decoder_prefill_tf32, with every
+ * projection one kllm_gemm_w8 (int8 weights x 24-bit fixed-point activations, exact integer products on the
+ * tcgen05 kind::i8 tensor cores) and the last position's classifier through the int8 GEMV.  KV-cache rows and
+ * logits agree with the position-by-position path within the north-star tolerance (|dlogit| <= 1e-4,
+ * tests/test_prefill_w8_gpu.py), NOT bit for bit.  group_size 64 on one GPU with dim, hidden_dim and
+ * head_num * head_size multiples of 64; KLLM_E_UNSUPPORTED otherwise (fp32: kllm_decoder_prefill_tf32). */
+int kllm_decoder_prefill_w8(kllm_decoder* dec, const int32_t* tokens_host, int32_t n_tokens, int32_t start_pos,
+                            int32_t* next_host);
 /* Device-resident greedy loop: positions start_pos .. start_pos+n_steps-1, each step feeding
  * the previous argmax back without leaving the GPU; ids copied to out_tokens_host at the end
  * (one synchronisation).  teacher_host (optional, n_steps ids) forces the inputs instead. */

@@ -83,6 +83,7 @@ _SIGNATURES = {
     "kllm_argmax_f32_sync": (c_int64, [c_void_p, c_int64, c_void_p]),
     "kllm_gemv_fused": (c_int, [POINTER(GemvJob), c_void_p]),
     "kllm_gemm_tf32": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),
+    "kllm_gemm_w8": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),
     "kllm_comm_unique_id": (c_int, [c_void_p]),
     "kllm_comm_create": (c_int, [c_int, c_int, c_int, c_int, c_void_p, POINTER(c_void_p)]),
     "kllm_comm_ipc_handle": (c_int, [c_void_p, c_void_p]),
@@ -96,6 +97,7 @@ _SIGNATURES = {
     "kllm_decoder_step": (c_int, [c_void_p, c_int32, c_int32, c_int, POINTER(c_int32)]),
     "kllm_decoder_prompt": (c_int, [c_void_p, POINTER(c_int32), c_int32, c_int32, POINTER(c_int32)]),
     "kllm_decoder_prefill_tf32": (c_int, [c_void_p, POINTER(c_int32), c_int32, c_int32, POINTER(c_int32)]),
+    "kllm_decoder_prefill_w8": (c_int, [c_void_p, POINTER(c_int32), c_int32, c_int32, POINTER(c_int32)]),
     "kllm_decoder_generate": (c_int, [c_void_p, c_int32, c_int32, c_int32, POINTER(c_int32),
                                       POINTER(c_int32)]),
     "kllm_decoder_logits": (c_int, [c_void_p, c_void_p]),

@@ -128,6 +128,7 @@ struct kllm_decoder {
   // batched tcgen05 prefill (kllm_decoder_prefill_tf32): activations of one block of prompt positions
   float* pf_buf = nullptr;
   PrefillWorkspace pf_ws{};
+  void* pf_w8_ws = nullptr;  // kllm_decoder_prefill_w8: kllm_gemm_w8's activation workspace
 };
 
 namespace {
@@ -430,6 +431,7 @@ void kllm_decoder_destroy(kllm_decoder* dc) {
   if (dc->out_tokens) cudaFree(dc->out_tokens);
   if (dc->teacher) cudaFree(dc->teacher);
   if (dc->pf_buf) cudaFree(dc->pf_buf);
+  if (dc->pf_w8_ws) cudaFree(dc->pf_w8_ws);
   if (dc->st_host) cudaFreeHost(dc->st_host);
   if (dc->io_host) cudaFreeHost(dc->io_host);
   if (dc->own_stream && dc->stream) cudaStreamDestroy(dc->stream);
@@ -485,15 +487,22 @@ int kllm_decoder_prompt(kllm_decoder* dc, const int32_t* tokens_host, int32_t n_
   return 0;
 }
 
-int kllm_decoder_prefill_tf32(kllm_decoder* dc, const int32_t* tokens_host, int32_t n_tokens, int32_t start_pos,
-                              int32_t* next_host) {
-  if (!dc || !tokens_host || !next_host || n_tokens <= 0 || start_pos < 0) return KLLM_E_INVALID;
+}  // extern "C"
+
+namespace {
+
+// Batched prefill shared by kllm_decoder_prefill_tf32 (fp32 weights, kllm_gemm_tf32) and
+// kllm_decoder_prefill_w8 (int8 group-64 weights, kllm_gemm_w8); the callers check the checkpoint kind.
+int prefill_batched(kllm_decoder* dc, const int32_t* tokens_host, int32_t n_tokens, int32_t start_pos,
+                    int32_t* next_host, bool w8) {
+  constexpr int kBlock = 256;  // prompt positions per pass = the N of the tcgen05.mma (tf32)
   const kllm_decoder_desc& d = dc->d;
-  if (start_pos + n_tokens > d.seq_len) return KLLM_E_INVALID;
-  if (d.group_size != 0 || d.tp_size > 1) return KLLM_E_UNSUPPORTED;  // fp32 checkpoints, one GPU
-  constexpr int kBlock = 256;  // prompt positions per pass = the N of the tcgen05.mma
   const int hs = dc->head_size, q_rows = d.head_num * hs, kvd = dc->kv_dim;
-  if ((d.dim & 3) || (d.hidden_dim & 3) || (q_rows & 3)) return KLLM_E_UNSUPPORTED;
+  if (w8 && dc->pf_w8_ws == nullptr) {  // the GEMM's digit planes + steps for the widest input of a block
+    const size_t kmax = static_cast<size_t>(std::max(std::max(d.dim, d.hidden_dim), q_rows));
+    const size_t bytes = 3 * kBlock * kmax + 4 * (kmax / 64) * kBlock;
+    if (cudaMalloc(&dc->pf_w8_ws, bytes) != cudaSuccess) return static_cast<int>(cudaErrorMemoryAllocation);
+  }
   if (dc->pf_buf == nullptr) {
     const size_t per_row = static_cast<size_t>(3 * d.dim + 2 * q_rows + 2 * kvd + 2 * d.hidden_dim);
     if (cudaMalloc(&dc->pf_buf, per_row * kBlock * sizeof(float)) != cudaSuccess)
@@ -518,6 +527,11 @@ int kllm_decoder_prefill_tf32(kllm_decoder* dc, const int32_t* tokens_host, int3
   m.tok_emb = d.tok_emb, m.attn_norm = dc->attn_norm.data(), m.ffn_norm = dc->ffn_norm.data();
   m.wq = dc->wq.data(), m.wk = dc->wk.data(), m.wv = dc->wv.data(), m.wo = dc->wo.data();
   m.w1 = dc->w1.data(), m.w2 = dc->w2.data(), m.w3 = dc->w3.data();
+  if (w8) {
+    m.sq = dc->sq.data(), m.sk = dc->sk.data(), m.sv = dc->sv.data(), m.so = dc->so.data();
+    m.s1 = dc->s1.data(), m.s2 = dc->s2.data(), m.s3 = dc->s3.data();
+    m.w8_workspace = dc->pf_w8_ws;
+  }
   m.bq = dc->bq.empty() ? nullptr : dc->bq.data();
   m.bk = dc->bk.empty() ? nullptr : dc->bk.data();
   m.bv = dc->bv.empty() ? nullptr : dc->bv.data();
@@ -545,8 +559,9 @@ int kllm_decoder_prefill_tf32(kllm_decoder* dc, const int32_t* tokens_host, int3
     j.norm_w = d.final_norm;
     j.norm_eps = flavour_eps(d.flavour);
     j.in_dim = d.dim;
+    j.group_size = d.group_size;
     j.n_seg = 1;
-    j.seg[0] = {d.wcls, nullptr, nullptr, dc->logits, d.vocab_size};
+    j.seg[0] = {d.wcls, d.group_size ? d.scls : nullptr, nullptr, dc->logits, d.vocab_size};
     KLLM_TRY(gemv_dispatch(&j, GemvExtra{}, dc->stream));
   }
   argmax_advance_kernel<<<1, 1024, 0, dc->stream>>>(dc->logits, d.vocab_size, dc->st, nullptr, nullptr, d.seq_len);
@@ -556,6 +571,32 @@ int kllm_decoder_prefill_tf32(kllm_decoder* dc, const int32_t* tokens_host, int3
   KLLM_TRY(cudaStreamSynchronize(dc->stream));
   *next_host = hs_state->next;
   return 0;
+}
+
+}  // namespace
+
+extern "C" {
+
+int kllm_decoder_prefill_tf32(kllm_decoder* dc, const int32_t* tokens_host, int32_t n_tokens, int32_t start_pos,
+                              int32_t* next_host) {
+  if (!dc || !tokens_host || !next_host || n_tokens <= 0 || start_pos < 0) return KLLM_E_INVALID;
+  const kllm_decoder_desc& d = dc->d;
+  if (start_pos + n_tokens > d.seq_len) return KLLM_E_INVALID;
+  if (d.group_size != 0 || d.tp_size > 1) return KLLM_E_UNSUPPORTED;  // fp32 checkpoints, one GPU
+  const int q_rows = d.head_num * dc->head_size;
+  if ((d.dim & 3) || (d.hidden_dim & 3) || (q_rows & 3)) return KLLM_E_UNSUPPORTED;
+  return prefill_batched(dc, tokens_host, n_tokens, start_pos, next_host, false);
+}
+
+int kllm_decoder_prefill_w8(kllm_decoder* dc, const int32_t* tokens_host, int32_t n_tokens, int32_t start_pos,
+                            int32_t* next_host) {
+  if (!dc || !tokens_host || !next_host || n_tokens <= 0 || start_pos < 0) return KLLM_E_INVALID;
+  const kllm_decoder_desc& d = dc->d;
+  if (start_pos + n_tokens > d.seq_len) return KLLM_E_INVALID;
+  if (d.group_size != 64 || d.tp_size > 1) return KLLM_E_UNSUPPORTED;  // int8 group-64 checkpoints, one GPU
+  const int q_rows = d.head_num * dc->head_size;
+  if ((d.dim % 64) || (d.hidden_dim % 64) || (q_rows % 64)) return KLLM_E_UNSUPPORTED;  // whole groups per row
+  return prefill_batched(dc, tokens_host, n_tokens, start_pos, next_host, true);
 }
 
 int kllm_decoder_generate(kllm_decoder* dc, int32_t first_token, int32_t start_pos,

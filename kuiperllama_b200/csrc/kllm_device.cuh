@@ -129,6 +129,30 @@ __device__ __forceinline__ void int8x4_to_float(uint32_t packed, float out[4]) {
   out[3] = __fsub_rn(__uint_as_float(__byte_perm(t, 0x4B000000u, 0x7653)), magic);
 }
 
+// Fixed-point form of one 64-element activation group for the int8 x int8 paths (the fast decode
+// mode's dp4a / mma.sync rows, megakernel.cu, and the kind::i8 prompt GEMM, prefill_gemm.cu):
+//     x_i ~= step * q_i,  step = gmax * 2^-22,  q_i = rint(x_i * (2^22 / gmax)),  |q_i| <= 2^22,
+// q_i split into three balanced base-256 digits, q = 65536 a2 + 256 a1 + a0, each in int8.  An all-zero
+// group has step 0 and digits 0.  This is the ONE definition both kernels use.
+__device__ __forceinline__ float w8_group_step(float gmax) { return gmax * (1.0f / 4194304.0f); }  // 2^-22
+__device__ __forceinline__ float w8_group_inv(float gmax) { return gmax > 0.f ? 4194304.0f / gmax : 0.f; }
+// four values -> one packed word (byte b = element b) of each digit plane
+__device__ __forceinline__ void w8_digits4(const float (&e)[4], float inv, uint32_t& p0, uint32_t& p1,
+                                           uint32_t& p2) {
+  p0 = 0, p1 = 0, p2 = 0;
+#pragma unroll
+  for (int b = 0; b < 4; ++b) {
+    const int qv = __float2int_rn(e[b] * inv);  // |qv| <= 2^22
+    const int a0 = ((qv + 128) & 255) - 128;    // balanced digits: qv = 65536 a2 + 256 a1 + a0
+    const int q1 = (qv - a0) >> 8;
+    const int a1 = ((q1 + 128) & 255) - 128;
+    const int a2 = (q1 - a1) >> 8;
+    p0 |= static_cast<uint32_t>(a0 & 255) << (8 * b);
+    p1 |= static_cast<uint32_t>(a1 & 255) << (8 * b);
+    p2 |= static_cast<uint32_t>(a2 & 255) << (8 * b);
+  }
+}
+
 // swiglu_kernel.cu:16-19: value = 1/(1+exp(-a)); (a*value)*b.  Written with plain operators
 // on purpose: the reference build contracts expf's final scale multiply with the "1.0f +"
 // (SASS: MUFU.EX2; FFMA r, s, e, 1.0), and the same source form makes nvcc do the same here.

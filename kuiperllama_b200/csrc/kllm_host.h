@@ -39,6 +39,7 @@ int launch_mha(PosArg pos, int head_num, int layer_index, int seq_len, int kv_di
 int comm_tagged_areas(kllm_comm* comm, unsigned long long** areas8, int* world, int* rank, int* stride);
 
 // prefill.cu: one block of T prompt positions through every layer with batched tcgen05 GEMMs
+// (kllm_gemm_tf32 for fp32 weights; kllm_gemm_w8 for int8 group-64 weights when sq..s3 are set)
 struct PrefillModel {
   int dim, hidden_dim, layer_num, head_num, kv_head_num, vocab_size, seq_len, head_size, flavour;
   int mega_layout;  // 1: the persistent engine's head-major K / V cache layout (megakernel.cu)
@@ -49,6 +50,10 @@ struct PrefillModel {
   const float* const* ffn_norm;
   const void* const* wq; const void* const* wk; const void* const* wv; const void* const* wo;
   const void* const* w1; const void* const* w2; const void* const* w3;
+  // int8 only (NULL for fp32): per-layer scales [rows, in / 64] and the GEMM's activation workspace
+  const float* const* sq; const float* const* sk; const float* const* sv; const float* const* so;
+  const float* const* s1; const float* const* s2; const float* const* s3;
+  void* w8_workspace;
   const float* const* bq; const float* const* bk; const float* const* bv;
   float* key_cache; float* value_cache;
   const float* sin_cache; const float* cos_cache;

@@ -618,8 +618,8 @@ __device__ __noinline__ void quantize_input_inplace(float* xs, int M, int tid) {
     }
     gmax = fmaxf(gmax, __shfl_xor_sync(kFull, gmax, 1));
     gmax = fmaxf(gmax, __shfl_xor_sync(kFull, gmax, 2));  // also orders: every lane of the group has read
-    const float step = gmax * (1.0f / 4194304.0f);      // 2^-22
-    const float inv = gmax > 0.f ? 4194304.0f / gmax : 0.f;
+    const float step = w8_group_step(gmax);
+    const float inv = w8_group_inv(gmax);
     __syncwarp();
     if (on) {
       const int g = qg >> 2, q = qg & 3;
@@ -631,18 +631,8 @@ __device__ __noinline__ void quantize_input_inplace(float* xs, int M, int tid) {
 #pragma unroll
       for (int j = 0; j < 4; ++j) {  // 4 elements -> one word of each digit plane, written at once
         const float e[4] = {v[j].x, v[j].y, v[j].z, v[j].w};
-        uint32_t p0 = 0, p1 = 0, p2 = 0;
-#pragma unroll
-        for (int b = 0; b < 4; ++b) {
-          const int qv = __float2int_rn(e[b] * inv);  // |qv| <= 2^22
-          const int a0 = ((qv + 128) & 255) - 128;    // balanced digits: qv = 65536 a2 + 256 a1 + a0
-          const int q1 = (qv - a0) >> 8;
-          const int a1 = ((q1 + 128) & 255) - 128;
-          const int a2 = (q1 - a1) >> 8;
-          p0 |= static_cast<uint32_t>(a0 & 255) << (8 * b);
-          p1 |= static_cast<uint32_t>(a1 & 255) << (8 * b);
-          p2 |= static_cast<uint32_t>(a2 & 255) << (8 * b);
-        }
+        uint32_t p0, p1, p2;
+        w8_digits4(e, inv, p0, p1, p2);  // kllm_device.cuh: the definition shared with the kind::i8 GEMM
         o0[j] = p0, o1[j] = p1, o2[j] = p2;
       }
       if (q == 0) *reinterpret_cast<float*>(gb + ((3u + odd) & 3u) * 64) = step;

@@ -11,7 +11,9 @@
 //
 // Because of TF32 (10 mantissa bits per operand) the cache rows and the final logits agree with the
 // position-by-position path to ~1e-3 relative, not bit for bit; tests/test_prefill_gpu.py states the
-// bound.  fp32 checkpoints, single GPU.
+// bound.  fp32 checkpoints, single GPU.  Int8 (group 64) checkpoints take kllm_gemm_w8 instead (int8 weights
+// x 24-bit fixed-point activations, exact integer products): within 1e-4 of the position-by-position path,
+// tests/test_prefill_w8_gpu.py.
 #include <cuda_runtime.h>
 
 #include <cfloat>
@@ -183,7 +185,9 @@ int prefill_block(const PrefillModel& m, PrefillWorkspace& ws, const int32_t* to
                   cudaStream_t s) {
   const int dim = m.dim, hid = m.hidden_dim, hs = m.head_size, heads = m.head_num, kvh = m.kv_head_num;
   const int q_rows = heads * hs, kvd = kvh * hs;
-  auto gemm = [&](const float* x, const void* w, float* out, int K, int N) {
+  const bool w8 = m.sq != nullptr;
+  auto gemm = [&](const float* x, const void* w, const float* const* scales, int l, float* out, int K, int N) {
+    if (w8) return kllm_gemm_w8(x, static_cast<const int8_t*>(w), scales[l], out, m.w8_workspace, T, K, N, s);
     return kllm_gemm_tf32(x, static_cast<const float*>(w), out, T, K, N, s);
   };
   auto count = [&]() {
@@ -198,9 +202,9 @@ int prefill_block(const PrefillModel& m, PrefillWorkspace& ws, const int32_t* to
     const size_t layer_off = static_cast<size_t>(l) * m.seq_len * kvd;
     rmsnorm_rows_kernel<<<T, 256, 0, s>>>(ws.x, m.attn_norm[l], ws.xn, dim, m.eps);
     PF_TRY(count());
-    PF_TRY(gemm(ws.xn, m.wq[l], ws.q, dim, q_rows));
-    PF_TRY(gemm(ws.xn, m.wk[l], ws.k, dim, kvd));
-    PF_TRY(gemm(ws.xn, m.wv[l], ws.v, dim, kvd));
+    PF_TRY(gemm(ws.xn, m.wq[l], m.sq, l, ws.q, dim, q_rows));
+    PF_TRY(gemm(ws.xn, m.wk[l], m.sk, l, ws.k, dim, kvd));
+    PF_TRY(gemm(ws.xn, m.wv[l], m.sv, l, ws.v, dim, kvd));
     if (m.bq != nullptr) {
       add_bias_rows_kernel<<<T, 256, 0, s>>>(ws.q, m.bq[l], q_rows);
       add_bias_rows_kernel<<<T, 256, 0, s>>>(ws.k, m.bk[l], kvd);
@@ -215,16 +219,16 @@ int prefill_block(const PrefillModel& m, PrefillWorkspace& ws, const int32_t* to
     attn_rows_kernel<<<dim3(heads, T), 128, sc_bytes, s>>>(ws.q, m.key_cache + layer_off, m.value_cache + layer_off,
                                                            ws.att, cl, heads, heads / kvh, start_pos);
     PF_TRY(count());
-    PF_TRY(gemm(ws.att, m.wo[l], ws.tmp, q_rows, dim));
+    PF_TRY(gemm(ws.att, m.wo[l], m.so, l, ws.tmp, q_rows, dim));
     add_rows_kernel<<<ew_grid, 256, 0, s>>>(ws.x, ws.tmp, static_cast<size_t>(T) * dim);
     PF_TRY(count());
     rmsnorm_rows_kernel<<<T, 256, 0, s>>>(ws.x, m.ffn_norm[l], ws.xn, dim, m.eps);
     PF_TRY(count());
-    PF_TRY(gemm(ws.xn, m.w1[l], ws.h1, dim, hid));
-    PF_TRY(gemm(ws.xn, m.w3[l], ws.h3, dim, hid));
+    PF_TRY(gemm(ws.xn, m.w1[l], m.s1, l, ws.h1, dim, hid));
+    PF_TRY(gemm(ws.xn, m.w3[l], m.s3, l, ws.h3, dim, hid));
     swiglu_rows_kernel<<<ew_grid, 256, 0, s>>>(ws.h1, ws.h3, static_cast<size_t>(T) * hid);
     PF_TRY(count());
-    PF_TRY(gemm(ws.h1, m.w2[l], ws.tmp, hid, dim));
+    PF_TRY(gemm(ws.h1, m.w2[l], m.s2, l, ws.tmp, hid, dim));
     add_rows_kernel<<<ew_grid, 256, 0, s>>>(ws.x, ws.tmp, static_cast<size_t>(T) * dim);
     PF_TRY(count());
   }

@@ -244,6 +244,16 @@ class Decoder:
               "kllm_decoder_prefill_tf32")
         return nxt.value
 
+    def prefill_w8(self, tokens, start_pos: int = 0) -> int:
+        """TOLERANCED batched prefill of an int8 (group 64) checkpoint on the tcgen05 kind::i8 tensor cores;
+        same contract as prompt(), logits within 1e-4 of it.  Raises KllmError for fp32 checkpoints."""
+        n = len(tokens)
+        arr = (ctypes.c_int32 * n)(*[int(t) for t in tokens])
+        nxt = ctypes.c_int32(-1)
+        check(self.lib.kllm_decoder_prefill_w8(self.handle, arr, n, start_pos, ctypes.byref(nxt)),
+              "kllm_decoder_prefill_w8")
+        return nxt.value
+
     def generate(self, first_token: int, start_pos: int, n_steps: int, teacher=None):
         out = (ctypes.c_int32 * n_steps)()
         tf = None
